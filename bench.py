@@ -152,7 +152,7 @@ def cpu_reference(steps, warmup, workload, max_seconds=60.0):
     cores = os.cpu_count() or 1
     jobs = min(64, cores)
     x = make_data(kind, n, synth.SEED + 1)
-    times, per = [], {}
+    times, per, outputs = [], {}, {}
     t_all = time.perf_counter()
     for it in range(warmup + steps):
         tot = 0.0
@@ -163,6 +163,7 @@ def cpu_reference(steps, warmup, workload, max_seconds=60.0):
             if it == 0:
                 assert np.array_equal(y, x)
             tot += te[0] + td[0]
+            outputs[label] = (s, y)
             if it >= warmup or it == warmup + steps - 1:
                 per[label] = {"encode_MBps": n / te[0] / 1e6, "decode_MBps": n / td[0] / 1e6, "MBps": 2 * n / (te[0] + td[0]) / 1e6, "compressed_bytes": int(len(s))}
         if it >= warmup:
@@ -174,7 +175,7 @@ def cpu_reference(steps, warmup, workload, max_seconds=60.0):
             "sample": "the whole workload (%d bytes of %s data, %d-byte blocks; %s), compress+decompress in memory, %d worker threads, %d timed step(s); "
                       "C++ restatement of kanzi-go (no Go toolchain in this image)"
                       % (n, kind, BLOCK, " and ".join("-t %s -e %s" % (p[1], p[2]) for p in passes), jobs, len(times)),
-            "ms_per_step": t * 1e3, "levels": per, "steps": len(times)}
+            "ms_per_step": t * 1e3, "levels": per, "steps": len(times), "outputs": outputs}
 
 
 def static_config(workload, passes, block, nblocks, n, world):
@@ -199,6 +200,25 @@ def workload_label(name):
         (" (BASELINE.json metric configuration)" if name == "silesia" else "")
 
 
+DUMP_BYTES = 48 << 20  # all arrays of --dump-outputs together, in float32
+DUMP_SEED = 0x44554D50
+
+
+def dump_outputs(directory, outputs):
+    """--dump-outputs: for every level, the stream the last timed step wrote (<label>_compressed) and the bytes it decoded from it
+    (<label>_decompressed), as float32 .npy files, and their lengths in bytes (<label>_sizes, float64). An array larger than its
+    share of DUMP_BYTES is written as its elements at a fixed, seeded sample of positions (sorted): two builds that compute the
+    same bytes write the same files."""
+    os.makedirs(directory, exist_ok=True)
+    cap = DUMP_BYTES // 4 // (2 * len(outputs))
+    for label, (compressed, decompressed) in outputs.items():
+        np.save(os.path.join(directory, label + "_sizes.npy"), np.array([len(compressed), len(decompressed)], dtype=np.float64))
+        for kind, a in (("compressed", compressed), ("decompressed", decompressed)):
+            if len(a) > cap:
+                a = a[np.sort(np.random.default_rng(DUMP_SEED).integers(0, len(a), cap))]
+            np.save(os.path.join(directory, "%s_%s.npy" % (label, kind)), np.asarray(a, dtype=np.float32))
+
+
 def emit(line):
     """Writes the one JSON line to the real stdout (fd 1 is pointed at stderr during the run so that library chatter such
     as "NCCL version ..." cannot end up in front of it)."""
@@ -219,6 +239,7 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--mode", default="auto", choices=["auto", "weak", "sharded"])
     ap.add_argument("--workload", default="silesia", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     passes, BLOCK, n, kind, METRIC = WORKLOADS[args.workload]
     NBLOCKS = (n + BLOCK - 1) // BLOCK
@@ -234,6 +255,8 @@ def main():
         # K steps and W warm-up steps as asked (every step = the whole workload, 2-3 s on the box's 64 cores); a wall-clock cap of 4 minutes keeps a
         # large K within "a few minutes" and is reported through `steps`
         r = cpu_reference(max(args.steps, 1), max(args.warmup, 1), args.workload, max_seconds=240.0)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": "MB/s", "n_gpus": args.gpus, "steps": r["steps"], "warmup": max(args.warmup, 1),
                 "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic",
                 "config": static_config(args.workload, passes, BLOCK, NBLOCKS, n, world), "levels": r["levels"],
@@ -395,6 +418,8 @@ def main():
     launches = sum(c.launch_count(reset=True) for c in ctxs)
     kern, stages = collect(args.steps)
     profiling(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {label: (d_cmp[i][:m[i]].cpu().numpy(), d_dec[i][:n].cpu().numpy()) for i, (label, _, _) in enumerate(P)})
 
     # ---------------- end-to-end pass through the host-buffer C ABI (pinned host memory) ----------------
     e2e_ms, e2e_wall_ms, e2e_steps = 0.0, 0.0, 0

@@ -15,24 +15,21 @@ def needs_build():
     if not os.path.exists(OUT):
         return True
     t = os.path.getmtime(OUT)
-    for root in (CSRC, os.path.join(HERE, "..", "include")):
+    for root in (CSRC, os.path.join(CSRC, "_gen"), os.path.join(HERE, "..", "include")):
         for f in os.listdir(root):
-            if f.endswith((".cu", ".cuh", ".h", ".cpp")) and os.path.getmtime(os.path.join(root, f)) > t:
+            if f.endswith((".cu", ".cuh", ".h", ".cpp", ".inc")) and os.path.getmtime(os.path.join(root, f)) > t:
                 return True
     return False
 
 
 def build(force=False, verbose=False):
-    # TEXT's static dictionary is a constant of the kanzi format: generated from the reference tree when it is there (csrc/_gen/)
-    try:
-        import importlib.util
+    # TEXT's static dictionary is a constant of the kanzi format: csrc/_gen/ is generated from tests/golden/text_dict_en_1024.txt
+    import importlib.util
 
-        spec = importlib.util.spec_from_file_location("kz_gen_text_dict", os.path.join(HERE, "gen_text_dict.py"))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        mod.main()
-    except Exception as e:  # the library then builds without the TEXT stage
-        sys.stderr.write("gen_text_dict: %s\n" % e)
+    spec = importlib.util.spec_from_file_location("kz_gen_text_dict", os.path.join(HERE, "gen_text_dict.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    mod.main()
     if not force and not needs_build():
         return OUT
     srcs = [os.path.join(CSRC, s) for s in SOURCES if os.path.exists(os.path.join(CSRC, s))]
@@ -45,7 +42,7 @@ def build(force=False, verbose=False):
         raise RuntimeError("nvcc failed")
     os.replace(tmp, OUT)
     with open(os.path.join(HERE, "ptxas_info.txt"), "w") as f:
-        f.write("".join(ln for ln in r.stderr.splitlines(True) if "Compile time" not in ln))  # registers / spills / smem per kernel, reproducible
+        f.write("".join(ln for ln in r.stderr.splitlines(True) if "Compile time" not in ln))  # registers / spills / smem per kernel of this build (git-ignored)
     return OUT
 
 

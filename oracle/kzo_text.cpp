@@ -5,8 +5,8 @@
 //   textCodec2: constructor :1137-1188, reset :1190-1223, Forward :1225-1398, expandDictionary :1400-1413, emitSymbols :1415-1487,
 //   emitWordIndex2 :1489-1511, Inverse :1513-1718, MaxEncodedLen :1720-1724; wrapper TextCodec.Forward/Inverse :549-592.
 // Encoding type 1 (textCodec1, used with the FPAQ / CM / TPAQ / ANS1 entropy codecs) is not restated.
-// The static dictionary (1024 English words, :96-185) is a format constant of the reference: it is extracted from the reference
-// tree into oracle/_ref/kzo_text_dict.inc at build time (oracle/gen_text_dict.py), never committed.
+// The static dictionary (1024 English words, :96-185) is a format constant of the reference: it is written from
+// tests/golden/text_dict_en_1024.txt into oracle/_ref/kzo_text_dict.inc at build time (oracle/gen_text_dict.py).
 // The dictionary map of the reference holds pointers into dictList; expandDictionary reallocates dictList so the map may point
 // to stale copies, but an entry is only modified right after its map slot has been cleared, so index semantics are equivalent.
 #include <algorithm>

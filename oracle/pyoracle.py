@@ -19,7 +19,7 @@ T_TEXT, T_MM, T_UTF, T_PACK, T_DNA, T_EXE = 10, 15, 17, 18, 19, 9  # oracle only
 
 
 def build(force=False):
-    # the TEXT codec's static dictionary is a format constant of the reference: extracted into oracle/_ref/ (not committed)
+    # the TEXT codec's static dictionary is a format constant of the reference: written from tests/golden/ into oracle/_ref/ (not committed)
     from . import gen_text_dict
 
     gen_text_dict.main()

@@ -49,6 +49,15 @@ def main():
     with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_tables.json"), "w") as f:
         json.dump(out, f, indent=0)
     print({k: (len(v) if hasattr(v, "__len__") else v) for k, v in out.items()})
+    # TEXT's static dictionary (transform/TextCodec.go, _TC_DICT_EN_1024), a constant of the format that the library and the oracle embed
+    # (kanzi-go_b200/gen_text_dict.py, oracle/gen_text_dict.py): one word per line, letters only, as createDictionary reads it
+    tc = open(os.path.join(REF, "transform/TextCodec.go"), encoding="utf-8").read()
+    letters = "".join(c for c in re.search(r"_TC_DICT_EN_1024\s*=\s*\[\]byte\(`([^`]*)`\)", tc).group(1) if c.isascii() and c.isalpha())
+    words = re.findall(r"[A-Z][a-z]*", letters)
+    assert len(words) == 1024 and "".join(words) == letters
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "text_dict_en_1024.txt"), "w") as f:
+        f.write("\n".join(words) + "\n")
+    print({"text_dict_en_1024": len(words)})
 
 
 if __name__ == "__main__":
